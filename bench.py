@@ -207,7 +207,7 @@ def sst_e2e(ffi, device, blks, plan, after, args, stream, barrier, max_over_rank
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        k = max(1, min(args.steps, 3))
+        k = args.steps
         dms_acc = 0.0
         for _ in range(k):
             rows, st, h2d, dms = step()
@@ -484,6 +484,36 @@ def parity_check(ffi, device, name, plan, dev_src, first_handle, sample_rows, st
     return info
 
 
+def dump_outputs(out_dir, outputs):
+    """--dump-outputs: the merged results of the last timed step of each workload, as a caller receives them, one float64
+    .npy per array.  An int64 array becomes <name>_hi (its signed upper 32 bits) and <name>_lo (its lower 32 bits), both
+    exact in float64.  Files: c3_keys, c3_key_null, c3_acc (one row per group, sorted by key; the accumulator words of
+    b2_agg_partials), c4_col<i>, c4_col<i>_null (the top rows in order), c5_checksum ([crc64, total_kvs, total_bytes])."""
+    import numpy as np
+    import torch
+    arrays = {}
+
+    def ints(name, t):
+        t = torch.as_tensor(t).to("cpu", torch.int64)
+        arrays[name + "_hi"], arrays[name + "_lo"] = (t >> 32).double(), (t & 0xFFFFFFFF).double()
+
+    for name, res in outputs.items():
+        if name == "c3":
+            keys, nul, acc = res
+            ints("c3_keys", keys)
+            arrays["c3_key_null"] = nul.double().cpu()
+            ints("c3_acc", acc)
+        elif name == "c4":
+            for i, (c, n) in enumerate(zip(*res)):
+                ints(f"c4_col{i}", c)
+                arrays[f"c4_col{i}_null"] = n.double().cpu()
+        elif name == "c5":
+            ints("c5_checksum", [v - (1 << 64) if v >= 1 << 63 else v for v in res])
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a.numpy())
+
+
 def peak_hbm():
     p = os.path.join(ROOT, "MEASURED_PEAKS.json")
     if os.path.exists(p):
@@ -501,8 +531,10 @@ def traffic_per_entry(kernel):
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
-    ap.add_argument("--steps", type=int, default=5)
+    ap.add_argument("--steps", type=int, default=5, help="timed steps of every timed loop")
     ap.add_argument("--warmup", type=int, default=3)
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write the results of the last timed step of each workload to DIR/<name>.npy (see dump_outputs)")
     ap.add_argument("--impl", default="ours", choices=["ours", "reference"])
     ap.add_argument("--rows", type=int, default=1_000_000_000, help="rows per GPU of the headline table")
     ap.add_argument("--blocks", type=int, default=16, help="CF_WRITE blocks (regions) per GPU of the headline table")
@@ -519,6 +551,10 @@ def main():
     ap.add_argument("--no-jit", action="store_true", help="generic kernels only")
     ap.add_argument("--only", default="", help="debug: run one workload (c2|c4|c5) as the headline shape")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.only == "c2"):
+        ap.error("--dump-outputs: only the CUDA path's aggregation, TopN and checksum results are dumped (C2 leaves its rows on the device)")
     args.warmup = max(args.warmup, 3) if args.impl == "ours" else args.warmup
 
     rank = int(os.environ.get("RANK", "0"))
@@ -677,6 +713,7 @@ def main():
     sampler.start()
     r = run_workload(head, dev_src, args.steps, args.warmup, args.chunk)
     r["steps"] = args.steps
+    outputs = {head: merged[head]} if head in merged else {}  # (the end-to-end requests below overwrite merged["c3"])
     value = args.rows * world / (r["ms_per_step"] / 1e3)
     out_bytes = r["rows_out"] * (8 * 8) + 8 * ((r["rows_out"] + 63) // 64) * 8 if head == "c2" else 0
     kname = {"c3": "scan_kernel<PM_AGG>", "c2": "scan_kernel<PM_SCAN>", "c4": "scan_kernel<PM_TOPN>", "c5": "scan_kernel<PM_CHECKSUM>"}[head]
@@ -716,7 +753,7 @@ def main():
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record(stream)
-        k = max(1, min(args.steps, 3))
+        k = args.steps
         for _ in range(k):
             r_e2e, st_e = run_dag(ffi, plan, table_range(), host_src, ffi.LOC_HOST, args.chunk, stream.cuda_stream, after)
         e1.record(stream)
@@ -748,7 +785,7 @@ def main():
             barrier()
             w0, w1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
             w0.record(stream)
-            kw = max(1, min(args.steps, 5))
+            kw = args.steps
             for _ in range(kw):
                 r_w, st_w = run_dag(ffi, plan, table_range(), _P, ffi.LOC_HOST, args.chunk, stream.cuda_stream, after)
             w1.record(stream)
@@ -778,8 +815,10 @@ def main():
                 if not args.no_parity:
                     parity[nm] = parity_check(ffi, device, nm, plans.get(nm), src2, rank * args.sub_rows + args.sub_rows // 3,
                                               min(args.parity_rows // 4 if nm == "c2" else args.parity_rows, args.sub_rows // 2), stream.cuda_stream)
-                rr = run_workload(nm, src2, min(args.steps, 10), 3, args.chunk)
-                rr["steps"] = min(args.steps, 10)
+                rr = run_workload(nm, src2, args.steps, 3, args.chunk)
+                rr["steps"] = args.steps
+                if nm in merged:
+                    outputs[nm] = merged[nm]
                 ob = rr["rows_out"] * 64 + 8 * ((rr["rows_out"] + 63) // 64) * 8 if nm == "c2" else 0
                 kb = ib2 if nm != "c5" else sum(b.key_bytes + b.val_bytes + 8 * b.block.n for b in blks2)
                 rf = roofline({"c2": "scan_kernel", "c4": "topn_kernel", "c5": "checksum_kernel"}[nm], kb, ob, rr, ne2)
@@ -813,6 +852,8 @@ def main():
         dist.destroy_process_group()
     if rank != 0:
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     sub_out = []
     for nm, rec in sub:
         if nm in cpu_sub:
